@@ -346,6 +346,40 @@ def run_reference(args):
 
 
 # ---------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path hands its caller, for comparing two builds output for output
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def fsm_record_words(ptr, n):
+    """A batch of jr_fsm_record as an (n, 8) uint32 array: group, hdr, id0, addr, tok0 lo/hi, stride lo/hi.  Split into
+    32-bit words, every field survives the float64 it is written as exactly."""
+    import numpy as np
+    if n == 0:
+        return np.zeros((0, 8), dtype=np.uint32)
+    words = np.ctypeslib.as_array(C.cast(ptr, C.POINTER(C.c_uint32)), shape=(n, C.sizeof(abi.FsmRecord) // 4))
+    return words.copy()
+
+
+def write_outputs(path, outputs):
+    """<path>/<name>.npy in float64 for every output (all values are integers below 2**53, so exact).  When the whole set
+    is over DUMP_LIMIT_BYTES, the rows of the largest array are sampled: a seeded choice, kept in their original order,
+    whose row numbers are written as <name>_rows.npy."""
+    import numpy as np
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in outputs.items()}
+    budget = DUMP_LIMIT_BYTES - 4096 * (len(arrays) + 1)          # (room for the .npy headers)
+    if sum(a.nbytes for a in arrays.values()) > budget:
+        name = max(arrays, key=lambda k: arrays[k].nbytes)
+        a = arrays.pop(name)
+        keep = (budget - sum(b.nbytes for b in arrays.values())) // (a.nbytes // len(a) + 8)   # a row + its row number
+        rows = np.sort(np.random.default_rng(SEED).choice(len(a), size=keep, replace=False))
+        arrays[name], arrays[name + "_rows"] = a[rows], rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
+# ---------------------------------------------------------------------------------------------
 # GPU arms
 
 class Bench:
@@ -405,7 +439,7 @@ class Bench:
         return float(t.item())
 
     # ---- device-resident: proposals generated in the kernel, Instruction stream drained every step
-    def device_resident(self, G, R, steps, warmup, announce=True, sampler=None, **eng_kw):
+    def device_resident(self, G, R, steps, warmup, announce=True, sampler=None, keep_outputs=False, **eng_kw):
         torch, dist = self.torch, self.dist
         S = TICKS_PER_STEP
         capture = os.environ.get("JR_BENCH_CAPTURE", "1") != "0"      # diagnostic A/B only; the reported runs capture
@@ -420,8 +454,9 @@ class Bench:
         totals = (C.c_uint64 * 3)()
         applied = (C.c_uint32 * (G * R))()
         outstanding = [0]
+        outputs = {}
 
-        def take():
+        def take(keep=False):
             # device-resident leg: the batch must have LANDED in pinned host memory, but it is not walked here (the
             # end-to-end leg folds every record; doing it here as well would make this leg measure the host)
             ptr, batch = C.POINTER(abi.FsmRecord)(), abi.FsmBatch()
@@ -430,6 +465,9 @@ class Bench:
             totals[0] += batch.n_instructions
             totals[2] += batch.n_records
             outstanding[0] -= 1
+            if keep:       # copied out of the engine's staging buffer, which a later jr_fsm_records_async reuses
+                outputs["fsm_records"] = fsm_record_words(ptr, batch.n_records)
+                outputs["fsm_batch"] = [batch.n_records, batch.n_dropped, batch.n_instructions, *batch.node_offset]
 
         def one_step():
             if world > 1 and announce and announce_done[0] is not None:
@@ -479,7 +517,7 @@ class Bench:
             b.record(self.stream)
             evs.append((a, b))
         while outstanding[0]:
-            take()
+            take(keep=keep_outputs and capture and outstanding[0] == 1)      # the last batch is the last timed step's
         self.barrier()
         clocks = sampler.window(t0, time.time()) if sampler else None
         per = [a.elapsed_time(b) for a, b in evs]
@@ -504,6 +542,9 @@ class Bench:
                "faulted_replicas": faults, "commit_min": commit_min, "instructions": int(totals[0] + totals[1]),
                "records": int(totals[2]), "collective_us": collective_us, "clocks": clocks,
                "ms_per_step_rank_median": statistics.median(per)}
+        if keep_outputs:
+            outputs["leader_table"] = table
+            res["outputs"] = outputs
         del eng
         torch.cuda.empty_cache()
         return res
@@ -805,6 +846,9 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-others", action="store_true", help="skip configs #2/#4/#5 and the variants")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the headline arm's last timed step returned (its Instruction-record batch and the "
+                         "leader table after it; rank 0's shard) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -819,7 +863,10 @@ def main():
         sampler.start()
 
     # ---------------- headline: config #3, device resident ----------------
-    main_res = bn.device_resident(G, R, args.steps, max(args.warmup, 20), sampler=sampler)   # >= 20 untimed steps: also nvidia-smi's start-up
+    main_res = bn.device_resident(G, R, args.steps, max(args.warmup, 20), sampler=sampler,   # >= 20 untimed steps: also nvidia-smi's start-up
+                                  keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, main_res.pop("outputs"))
     clocks = main_res.pop("clocks")
     value, ms = main_res["value"], main_res["ms_total"]
     launches = args.steps * (6 + (1 if world > 1 else 0))   # sym2_kernel, step_kernel, truncate_kernel, fsm count / scan / pack (+ leader_table_kernel); the copy-out is a DMA

@@ -3,6 +3,7 @@
 import ctypes as C
 import os
 import re
+import shutil
 import subprocess
 
 import pytest
@@ -59,7 +60,9 @@ def test_election_timeout_is_the_same_function_everywhere(engine_lib, oracle_lib
 
 
 def test_engine_library_is_sm100a_cuda(engine_lib):
-    out = subprocess.run(["cuobjdump", "-lelf", ENGINE_LIB_PATH], capture_output=True, text=True).stdout
+    # the toolkit build() compiled with, when it is not on PATH
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.path.dirname(os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", ENGINE_LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out, out
 
 
