@@ -97,7 +97,7 @@ __global__ void __launch_bounds__(32 * R, step_min_ctas(R)) step_kernel(const De
       __syncthreads();
     }
   }
-  if (p0.symblk && p0.symblk[blk]) {   // every group of this block was folded by sym_kernel: only keep the hand-over chain alive
+  if (p0.symblk && p0.symblk[blk]) {   // every group of this block was folded by sym2_kernel: only keep the hand-over chain alive
     if (p0.n_parts > 1 && part + 1 < p0.n_parts && threadIdx.x == 0) st_release_u32(d.done + blk, p0.epoch + part + 1);
     return;
   }
@@ -550,7 +550,6 @@ constexpr uint32_t SCAN_THREADS = 1024;
 struct FsmHeader {          // written by fsm_pack_kernel next to the records
   unsigned long long n_records, n_dropped, n_instructions;
   uint32_t node_offset[JR_MAX_REPLICAS + 1];
-  uint32_t ready;           // epoch of the batch, written last
 };
 
 // Three small kernels (CTAs of T threads; the CPU emulation runs them with T = 1):
@@ -687,19 +686,6 @@ __global__ void fsm_pack_kernel(const Dev d, const unsigned long long* part, Fsm
   }
 }
 
-// Packed batch (device) -> the engine's pinned host buffer, by the SMs: the size is only known on the device, so
-// a cudaMemcpyAsync would need a host round trip first.  Runs on the copy-out stream next to the following step.
-__global__ void fsm_copy_kernel(const uint4* __restrict__ src, const FsmHeader* __restrict__ hdr, uint4* __restrict__ dst,
-                                FsmHeader* hdr_dst, uint32_t epoch) {
-  const size_t n = (size_t)hdr->n_records * 2;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) dst[i] = src[i];
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
-    FsmHeader h = *hdr;
-    h.ready = epoch;
-    *hdr_dst = h;
-  }
-}
-
 __global__ void max_u32_kernel(const uint32_t* v, size_t n, uint32_t* out) {
   uint32_t m = 0;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
@@ -780,7 +766,7 @@ struct jr_engine {
   void* many_buf = nullptr;
   size_t many_cap = 0;
   // Instruction-stream drain (JR_F_CAPTURE_FSM): scan -> pack into stage[b] on the engine stream, then
-  // fsm_copy_kernel moves stage[b] into the pinned host buffer host[b] on the d2h stream.
+  // the copy engine moves stage[b] into the pinned host buffer host[b] on the d2h stream.
   unsigned long long* fsm_part = nullptr;                     // device, 3 x (CTAs of the count/pack kernels): per-CTA sums -> offsets
   uint32_t fsm_cap = 0;                                       // records per batch
   uint4* fsm_stage[NBUF] = {nullptr, nullptr};                // device, 2 * fsm_cap uint4 each
@@ -791,20 +777,15 @@ struct jr_engine {
   cudaEvent_t fsm_landed[NBUF] = {nullptr, nullptr};          // copy into host[b] finished (d2h stream)
   size_t fsm_copied[NBUF] = {0, 0};                           // records of stage[b] the enqueued copy covers
   size_t fsm_last_records = 0;                                // size of the last batch taken (the next copy's guess)
-  int fsm_copy_by_sm = 0;                                     // JR_FSM_COPY=sm (A/B): fsm_copy_kernel instead of the copy engine
   bool fsm_used[NBUF] = {false, false};
   int fsm_i = 0, fsm_pending[NBUF] = {0, 0}, fsm_npending = 0;
   std::mutex qmu;   // the two FIFOs of outstanding copy-outs (fsm_pending, tab_pending) and fsm_last_records: a second host thread may
                     // sit in jr_fsm_records_wait / jr_leader_table_wait while the first one keeps submitting
-  uint32_t fsm_epoch = 0;
   // symmetric-group fold
   uint8_t* symdone = nullptr;   // device, Gp entries
   uint8_t* symblk = nullptr;    // device, Gp / 32 entries
   bool auto_trunc = false;      // jr_set_auto_truncate
   uint32_t auto_trunc_margin = 0;
-  int no_fold = 0;              // JR_NO_FOLD=1 (A/B, tests)
-  int no_parts_hint = 0;        // JR_NO_PARTS_HINT=1 (A/B): always cut step_kernel's grid in parts, even while the fold takes every group
-  int sym_one_lane = 0;         // JR_SYM_ONE_LANE=1 (A/B, tests): sym_kernel (one lane per group) instead of sym2_kernel
   uint64_t launches_folded = 0;
   bool last_launch_folded = false;
 };
@@ -902,20 +883,16 @@ static jr_status launch_step(jr_engine* e, const StepParams& p_in) {
 
 template <int R>
 static void launch_sym_r(jr_engine* e, const StepParams& p) {
-  if constexpr (R >= 2) {
-    if (e->sym_one_lane)
-      JR_LAUNCH(sym_kernel<R>, (e->d.Gp + SYM_LANES - 1) / SYM_LANES, SYM_LANES, e->stream, e->d, p, e->symdone);
-    else
-      JR_LAUNCH_SMEM(sym2_kernel<R>, (e->d.Gp + SYM2_GROUPS - 1) / SYM2_GROUPS, 2 * SYM2_GROUPS,
-                     (size_t)SYM2_UNITS * SYM2_GROUPS * sizeof(uint4), e->stream, e->d, p, e->symdone, e->symblk);
-  }
+  if constexpr (R >= 2)
+    JR_LAUNCH_SMEM(sym2_kernel<R>, (e->d.Gp + SYM2_GROUPS - 1) / SYM2_GROUPS, 2 * SYM2_GROUPS,
+                   (size_t)SYM2_UNITS * SYM2_GROUPS * sizeof(uint4), e->stream, e->d, p, e->symdone, e->symblk);
 }
 
 // May this launch be offered to the symmetric-group fold?  (Whether a GROUP takes it is sym_enter's decision.)
 static bool fold_eligible(const jr_engine* e, const StepParams& p) {
   const Dev& d = e->d;
   const uint32_t whole = PH_RESET_OUT | PH_DRAIN | PH_TICK;
-  if (e->no_fold || (d.flags & (JR_F_STREAM_DIGEST | JR_F_SLED_COMMIT_KEY_STRICT | JR_F_NO_SYMMETRIC_FOLD))) return false;
+  if (d.flags & (JR_F_STREAM_DIGEST | JR_F_SLED_COMMIT_KEY_STRICT | JR_F_NO_SYMMETRIC_FOLD)) return false;
   if (d.R < 2 || d.U < d.R + 7 || d.resident != 0xffu || p.dt == 0) return false;
   if ((p.phases & ~(uint32_t)PH_PROPOSE) != whole || p.n_ticks < 2) return false;
   if (p.proposals && p.prop_stride != d.G) return false;
@@ -930,10 +907,6 @@ static jr_status launch_step_once(jr_engine* e, const StepParams& p_in) {
   if (fold_eligible(e, p)) {
     DISPATCH_R(e->cfg.n_replicas, (launch_sym_r<RR>(e, p)));
     CK(cudaGetLastError());
-    if (e->sym_one_lane) {   // (sym2_kernel writes symblk itself)
-      JR_LAUNCH(sym_blocks_kernel, (n_blocks + 127) / 128, 128, e->stream, e->symdone, e->symblk, n_blocks);
-      CK(cudaGetLastError());
-    }
     p.symdone = e->symdone;
     p.symblk = e->symblk;
     e->launches_folded += 1;
@@ -943,8 +916,8 @@ static jr_status launch_step_once(jr_engine* e, const StepParams& p_in) {
   // When the fold has been taking every group (no launch of the last two left one behind -- a hint the kernel stores in
   // mapped host memory), step_kernel's CTAs only look at symblk and return: do not cut them in parts, which would cost
   // each of them a ticket and two barriers first.  A wrong guess costs balance in that one launch, nothing else.
-  if (p.symdone && !e->sym_one_lane && e->h_unfolded && (*e->h_unfolded == 0 || p.epoch - *e->h_unfolded > 2u * 8u) && !e->force_parts)
-    if (!e->no_parts_hint) p.n_parts = 1;
+  if (p.symdone && e->h_unfolded && (*e->h_unfolded == 0 || p.epoch - *e->h_unfolded > 2u * 8u) && !e->force_parts)
+    p.n_parts = 1;
   p.part_ticks = (p.n_ticks + p.n_parts - 1) / p.n_parts;
   p.n_parts = (p.n_ticks + p.part_ticks - 1) / p.part_ticks;  // no empty trailing part
   p.n_blocks = n_blocks;
@@ -957,8 +930,7 @@ static jr_status launch_step_once(jr_engine* e, const StepParams& p_in) {
   DISPATCH_R(e->cfg.n_replicas, (launch_step_r<RR>(e, p, sorted, grid, smem)));
   CK(cudaGetLastError());
   if (p.trunc) {   // sym2_kernel truncated the groups it folded
-    JR_LAUNCH(truncate_kernel, (e->d.Gp + 127) / 128, 128, e->stream, e->d, p.trunc_margin,
-              (const uint8_t*)((p.symdone && !e->sym_one_lane) ? p.symdone : nullptr));
+    JR_LAUNCH(truncate_kernel, (e->d.Gp + 127) / 128, 128, e->stream, e->d, p.trunc_margin, p.symdone);
     CK(cudaGetLastError());
   }
   e->launches_sorted += sorted ? 1 : 0;
@@ -1119,10 +1091,6 @@ jr_status jr_engine_create(const jr_config* cfg, jr_engine** out) {
     if (aerr == cudaSuccess) aerr = cudaHostAlloc((void**)&e->h_unfolded, sizeof(uint32_t), cudaHostAllocMapped);
     if (aerr == cudaSuccess) *e->h_unfolded = 0;
     if (aerr == cudaSuccess) aerr = cudaHostGetDevicePointer((void**)&e->d.hunf, (void*)e->h_unfolded, 0);
-    if (const char* ev = getenv("JR_NO_FOLD")) e->no_fold = atoi(ev);
-    if (const char* ev = getenv("JR_SYM_ONE_LANE")) e->sym_one_lane = atoi(ev);
-    if (const char* ev = getenv("JR_NO_PARTS_HINT")) e->no_parts_hint = atoi(ev);
-    if (const char* ev = getenv("JR_FSM_COPY")) e->fsm_copy_by_sm = strcmp(ev, "sm") == 0;
     if (const char* ev = getenv("JR_PARTS")) e->force_parts = (uint32_t)std::min(std::max(atoi(ev), 0), 8);
 #ifndef JR_EMU
     if (aerr == cudaSuccess) {
@@ -1320,7 +1288,6 @@ static jr_status fsm_records_enqueue(jr_engine* e) {
   e->fsm_i = (b + 1) % jr_engine::NBUF;
   const size_t plane = (size_t)d.R * d.Gp;
   if (e->fsm_used[b]) CK(cudaStreamWaitEvent(e->stream, e->fsm_landed[b], 0));  // stage[b] has left the device
-  const uint32_t epoch = ++e->fsm_epoch;
 #ifdef JR_EMU
   const uint32_t T = 1, Ts = 1;
 #else
@@ -1335,20 +1302,14 @@ static jr_status fsm_records_enqueue(jr_engine* e) {
   CK(cudaGetLastError());
   CK(cudaEventRecord(e->fsm_packed[b], e->stream));
   CK(cudaStreamWaitEvent(e->d2h, e->fsm_packed[b], 0));
-  if (e->fsm_copy_by_sm) {
-    JR_LAUNCH(fsm_copy_kernel, 32, 256, e->d2h, e->fsm_stage[b], e->fsm_stage_hdr[b], e->fsm_host[b], e->fsm_host_hdr[b], epoch);
-    CK(cudaGetLastError());
-    e->fsm_copied[b] = e->fsm_cap;
-  } else {
-    // Copy engine, speculatively: the batch size is only known on the device, so copy as many records as the previous
-    // batch held plus a margin; fsm_records_take fetches the rest in the (rare) case the batch turned out larger.
-    // (fsm_copy_kernel's stores to host memory share LSUs with the next step's kernel: one wave of CTAs, so the
-    // slowest SM sets its duration.  A DMA copy takes nothing from the SMs.)
-    const size_t guess = std::min<size_t>(e->fsm_cap, std::max<size_t>(last_records + last_records / 8 + 1024, 16384));
-    if (guess) CK(cudaMemcpyAsync(e->fsm_host[b], e->fsm_stage[b], guess * sizeof(jr_fsm_record), cudaMemcpyDeviceToHost, e->d2h));
-    CK(cudaMemcpyAsync(e->fsm_host_hdr[b], e->fsm_stage_hdr[b], sizeof(FsmHeader), cudaMemcpyDeviceToHost, e->d2h));
-    e->fsm_copied[b] = guess;
-  }
+  // Copy engine, speculatively: the batch size is only known on the device, so copy as many records as the previous
+  // batch held plus a margin; fsm_records_take fetches the rest in the (rare) case the batch turned out larger.
+  // (A copy by the SMs would store to host memory through the LSUs the next step's kernel needs: that kernel is one wave
+  // of CTAs, so the slowest SM sets its duration.  A DMA copy takes nothing from the SMs.)
+  const size_t guess = std::min<size_t>(e->fsm_cap, std::max<size_t>(last_records + last_records / 8 + 1024, 16384));
+  if (guess) CK(cudaMemcpyAsync(e->fsm_host[b], e->fsm_stage[b], guess * sizeof(jr_fsm_record), cudaMemcpyDeviceToHost, e->d2h));
+  CK(cudaMemcpyAsync(e->fsm_host_hdr[b], e->fsm_stage_hdr[b], sizeof(FsmHeader), cudaMemcpyDeviceToHost, e->d2h));
+  e->fsm_copied[b] = guess;
   CK(cudaEventRecord(e->fsm_landed[b], e->d2h));
   e->fsm_used[b] = true;
   std::lock_guard<std::mutex> l(e->qmu);
@@ -1542,28 +1503,39 @@ jr_status jr_step(jr_engine* e, jr_step_args* a) {
   return ovf ? JR_E_CAPACITY : JR_OK;
 }
 
+// One fused run of n_steps whole ticks from where the engine stands (jr_run and the batched calls).  `src` carries the
+// proposal source only (n_synth, proposals / prop_stride or tok_runs / tok_route); everything else comes from the engine
+// and the arguments.  Instructions accumulate until drained.  b >= 0: the batch slot the run reads, released once the
+// run has finished with it.
+static jr_status fused_run(jr_engine* e, const StepParams& src, uint64_t now0, uint32_t dt, uint32_t n_steps, int b) {
+  StepParams p = src;
+  p.now = now0;
+  p.dt = dt;
+  p.n_ticks = n_steps;
+  p.step_index = e->step_index;
+  p.cur = e->cur;
+  p.phases = PH_RESET_OUT | PH_DRAIN | ((p.n_synth || p.proposals || p.tok_runs) ? PH_PROPOSE : 0u) | PH_TICK;
+  p.trunc = e->auto_trunc ? 1u : 0u;
+  p.trunc_margin = e->auto_trunc_margin;
+  jr_status st = launch_step(e, p);
+  if (st != JR_OK) return st;
+  if (b >= 0) {
+    CK(cudaEventRecord(e->batch_free[b], e->stream));
+    e->batch_used[b] = true;
+  }
+  e->cur ^= (int)(n_steps & 1u);
+  e->step_index += n_steps;
+  return JR_OK;
+}
+
 jr_status jr_run(jr_engine* e, uint64_t now0, uint32_t dt, uint32_t n_steps, uint32_t n_synth) {
   if (!e) return JR_E_INVAL;
   if (n_synth > 8) { set_err("n_synth <= 8"); return JR_E_INVAL; }
   CK(cudaSetDevice(e->cfg.device));
   if (n_steps == 0) return JR_OK;
-  StepParams p;
-  p.now = now0;
-  p.step_index = e->step_index;
-  p.n_synth = n_synth;
-  p.n_ticks = n_steps;
-  p.dt = dt;
-  p.cur = e->cur;
-  p.proposals = nullptr;
-  p.prop_stride = 0;
-  p.phases = PH_RESET_OUT | PH_DRAIN | (n_synth ? PH_PROPOSE : 0u) | PH_TICK;   // Instructions accumulate until drained
-  p.trunc = e->auto_trunc ? 1u : 0u;
-  p.trunc_margin = e->auto_trunc_margin;
-  jr_status st = launch_step(e, p);
-  if (st != JR_OK) return st;
-  e->cur ^= (int)(n_steps & 1u);
-  e->step_index += n_steps;
-  return JR_OK;
+  StepParams src{};
+  src.n_synth = n_synth;
+  return fused_run(e, src, now0, dt, n_steps, -1);
 }
 
 // Grow batch[b] to n entries once its last reader is done; returns with the h2d stream fenced on that reader.
@@ -1577,29 +1549,6 @@ static jr_status batch_reserve(jr_engine* e, int b, size_t n) {
     CK(cudaMalloc(&e->batch[b], n * sizeof(jr_proposal)));
     e->batch_cap[b] = n;
   }
-  return JR_OK;
-}
-
-// The fused launch over batch[b] (already ordered after whatever filled it on e->stream).
-static jr_status batch_launch(jr_engine* e, int b, uint64_t now0, uint32_t dt, uint32_t n_steps) {
-  StepParams p;
-  p.now = now0;
-  p.step_index = e->step_index;
-  p.n_synth = 0;
-  p.n_ticks = n_steps;
-  p.dt = dt;
-  p.cur = e->cur;
-  p.proposals = e->batch[b];
-  p.prop_stride = e->d.G;
-  p.phases = PH_RESET_OUT | PH_DRAIN | PH_PROPOSE | PH_TICK;
-  p.trunc = e->auto_trunc ? 1u : 0u;
-  p.trunc_margin = e->auto_trunc_margin;
-  jr_status st = launch_step(e, p);
-  if (st != JR_OK) return st;
-  CK(cudaEventRecord(e->batch_free[b], e->stream));
-  e->batch_used[b] = true;
-  e->cur ^= (int)(n_steps & 1u);
-  e->step_index += n_steps;
   return JR_OK;
 }
 
@@ -1620,7 +1569,10 @@ jr_status jr_run_proposals(jr_engine* e, uint64_t now0, uint32_t dt, uint32_t n_
   CK(cudaMemcpyAsync(e->batch[b], proposals, n * sizeof(jr_proposal), cudaMemcpyHostToDevice, e->h2d));
   CK(cudaEventRecord(e->batch_ready[b], e->h2d));
   CK(cudaStreamWaitEvent(e->stream, e->batch_ready[b], 0));
-  return batch_launch(e, b, now0, dt, n_steps);
+  StepParams src{};
+  src.proposals = e->batch[b];
+  src.prop_stride = G;
+  return fused_run(e, src, now0, dt, n_steps, b);
 }
 
 jr_status jr_run_tokens(jr_engine* e, uint64_t now0, uint32_t dt, uint32_t n_steps, const uint64_t* tokens) {
@@ -1648,7 +1600,10 @@ jr_status jr_run_tokens(jr_engine* e, uint64_t now0, uint32_t dt, uint32_t n_ste
   const unsigned blocks = (unsigned)std::min<size_t>((n + 255) / 256, (size_t)148 * 16);
   JR_LAUNCH(route_tokens_kernel, blocks, 256, e->stream, e->tokbuf[b], e->route, e->batch[b], G, n);
   CK(cudaGetLastError());
-  return batch_launch(e, b, now0, dt, n_steps);
+  StepParams src{};
+  src.proposals = e->batch[b];
+  src.prop_stride = G;
+  return fused_run(e, src, now0, dt, n_steps, b);
 }
 
 jr_status jr_run_token_runs(jr_engine* e, uint64_t now0, uint32_t dt, uint32_t n_steps, const jr_token_run* runs) {
@@ -1663,28 +1618,10 @@ jr_status jr_run_token_runs(jr_engine* e, uint64_t now0, uint32_t dt, uint32_t n
   CK(cudaMemcpyAsync(e->batch[b], runs, (size_t)G * sizeof(jr_token_run), cudaMemcpyHostToDevice, e->h2d));
   CK(cudaEventRecord(e->batch_ready[b], e->h2d));
   CK(cudaStreamWaitEvent(e->stream, e->batch_ready[b], 0));
-  StepParams p;
-  p.now = now0;
-  p.step_index = e->step_index;
-  p.n_synth = 0;
-  p.n_ticks = n_steps;
-  p.dt = dt;
-  p.cur = e->cur;
-  p.proposals = nullptr;
-  p.prop_stride = 0;
-  p.tok_runs = reinterpret_cast<const uint4*>(e->batch[b]);
-  p.tok_route = e->route;    // on the engine stream: ordered after the leader_table_kernel that last wrote it
-  p.tok_tick = 0;
-  p.phases = PH_RESET_OUT | PH_DRAIN | PH_PROPOSE | PH_TICK;
-  p.trunc = e->auto_trunc ? 1u : 0u;
-  p.trunc_margin = e->auto_trunc_margin;
-  st = launch_step(e, p);
-  if (st != JR_OK) return st;
-  CK(cudaEventRecord(e->batch_free[b], e->stream));
-  e->batch_used[b] = true;
-  e->cur ^= (int)(n_steps & 1u);
-  e->step_index += n_steps;
-  return JR_OK;
+  StepParams src{};
+  src.tok_runs = reinterpret_cast<const uint4*>(e->batch[b]);
+  src.tok_route = e->route;    // on the engine stream: ordered after the leader_table_kernel that last wrote it
+  return fused_run(e, src, now0, dt, n_steps, b);
 }
 
 jr_status jr_drain_fsm(jr_engine* e, jr_fsm_instr* out, size_t cap, size_t* n) {

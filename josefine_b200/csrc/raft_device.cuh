@@ -102,7 +102,7 @@ struct StepParams {
   uint32_t n_parts = 1, part_ticks = 0, n_blocks = 0, epoch = 0;
   uint32_t trunc = 0, trunc_margin = 0;   // jr_set_auto_truncate: this launch ends with jr_truncate(trunc_margin)
   uint32_t ticket_base = 0;      // value of the ticket counter when this launch starts (every CTA of a split launch takes exactly one)
-  // Symmetric-group fold (sym_fold.cuh): set when sym_kernel ran in front of this launch.  symdone[g] = 1: group g's
+  // Symmetric-group fold (sym_fold.cuh): set when sym2_kernel ran in front of this launch.  symdone[g] = 1: group g's
   // whole launch has been applied already; symblk[b] = 1: that holds for all 32 groups of block b.
   const uint8_t* symdone = nullptr;
   const uint8_t* symblk = nullptr;

@@ -1,25 +1,24 @@
-// sym_fold.cuh -- the symmetric-group fold: a whole fused launch of a group in TWO lanes (sym2_kernel), or in one
-// (sym_kernel, the first version: A/B and fallback, JR_SYM_ONE_LANE=1).
+// sym_fold.cuh -- the symmetric-group fold: a whole fused launch of a group in TWO lanes (sym2_kernel).
 //
 // In a healthy group every follower is in the same state: same term, same head and commit, the same mail from the
 // leader in flight, and the leader holds the same progress entry for each of them.  R-1 replicas then make the same
-// decisions on the same data, tick after tick.  These kernels exploit that symmetry exactly, not approximately:
+// decisions on the same data, tick after tick.  This kernel exploits that symmetry exactly, not approximately:
 // the leader's state and ONE follower state that stands for all R-1 followers, the mail between them in its canonical
 // shapes (listed below), and the very handlers of raft_device.cuh -- restated here for scalar operands, each citing
 // the same reference lines -- for all n ticks of the launch.  No mailboxes in HBM, no divergence between roles; what
 // is left is the data that really has to move: the proposal tokens in, the block-table rows of every replica and the
 // Instruction stream out.  sym2_kernel runs the two sides in two lanes of two warps (within a tick they only depend on
 // the previous tick's mail), with the mail, the row caches and the Instruction encoders in shared memory and one
-// barrier per tick; sym_kernel runs both in one lane with the mail in registers.
+// barrier per tick.
 //
 // Exactness contract:
-//   * Both FIRST CHECK that a group is symmetric, that its followers' tables agree over every id the launch can read,
+//   * It FIRST CHECKS that a group is symmetric, that its followers' tables agree over every id the launch can read,
 //     and that its mail in flight has the canonical shapes (sym_enter); every other group is left to step_kernel
 //     untouched.
 //   * If anything outside the canonical evolution would happen during the launch (a fault, an election timer that
-//     could fire, a HeartbeatResponse{has_committed: false}, a read below the compared rows, ...) the lane ABORTS (in
-//     sym2_kernel: tells the other lane through the mail, and both check the other's last mail after the last
-//     barrier): it has only written block-table rows and Instruction records beyond the FIFO counters, which
+//     could fire, a HeartbeatResponse{has_committed: false}, a read below the compared rows, ...) the lane ABORTS
+//     (tells the other lane through the mail, and both check the other's last mail after the last barrier): it has
+//     only written block-table rows and Instruction records beyond the FIFO counters, which
 //     step_kernel writes identically when it re-runs the group from the untouched state planes -- an abort costs time,
 //     never correctness.
 //   * On success the replicas' state planes, progress planes and the mailboxes of the last tick are written in the
@@ -42,7 +41,7 @@ namespace jr {
 struct SymMail {
   uint32_t hb, hb_commit;                 // leader -> followers
   uint32_t ae, ae_nb, ae_id[JR_MAX_AE_BLOCKS];
-  uint32_t mk;                            // the leader's largest block id when it sent this (sym2_kernel: which cache slots it may be rewriting)
+  uint32_t mk;                            // the leader's largest block id when it sent this (which cache slots it may be rewriting)
   uint32_t hbr, hbr_commit, hbr_has;      // followers -> leader
   uint32_t ar, ar_head;
 };
@@ -53,10 +52,6 @@ struct SymMail {
 // after the fill at entry no table READ leaves the SM (rows are still written through to HBM).  (A register shift
 // register cost ~400 instructions per tick in compare/select chains; local-memory arrays were slower still.)
 constexpr uint32_t SYM_ROWS = 8;
-#ifndef JR_SYM_LANES
-#define JR_SYM_LANES 128   // (A/B builds override it)
-#endif
-constexpr uint32_t SYM_LANES = JR_SYM_LANES;   // threads per CTA of sym_kernel: one warp per SM sub-partition
 // The Instruction streams are encoded AS THEY ARE PRODUCED, by the same streaming encoder fsm_flush uses (fsm_enc_push):
 // its state is parked in shared memory between two Instructions, [slot][lane] like the row caches.  (The raw FIFO +
 // fsm_flush round trip of step_kernel cost this kernel a quarter of its instructions and half of its DRAM traffic.)
@@ -66,7 +61,7 @@ constexpr uint32_t SYM_LANES = JR_SYM_LANES;   // threads per CTA of sym_kernel:
 // seq = seq0 + the lane's Instruction counter (lcnt / fcnt), which lives in a register anyway.
 constexpr uint32_t SYM_ENC_L = 5, SYM_ENC_F = 3;
 constexpr uint32_t SYM_SMEM_UNITS = 2 * SYM_ROWS + SYM_ENC_L + SYM_ENC_F;   // uint4 per lane
-// sym2_kernel: TWO lanes per group, in two warps of the same CTA -- one runs the leader's handlers, the other the
+// TWO lanes per group, in two warps of the same CTA -- one runs the leader's handlers, the other the
 // followers' -- because within a tick the two sides only depend on the mail of the PREVIOUS tick.  The kernel is latency
 // bound with 3.5 warps per SM sub-partition; this doubles the warps and halves each warp's serial chain.  The mail goes
 // through shared memory, double buffered, one __syncthreads() per tick:
@@ -75,12 +70,15 @@ constexpr uint32_t SYM_SMEM_UNITS = 2 * SYM_ROWS + SYM_ENC_L + SYM_ENC_F;   // u
 //                         flight; ids = 0: the follower lane derives them, see replicate())
 //   followers -> leader   C = {hbr | has << 1 | ar << 2 | abort << 8, hbr_commit, ar_head, -}
 constexpr uint32_t SYM2_GROUPS = 64;                                        // groups per CTA: 128 threads
+// CTAs per SM the launch bounds ask for: all 1,024 CTAs of 65,536 groups must be resident at once (a second wave would
+// double the time), so 7 per SM on 148 SMs, which holds the kernel to 72 registers per thread.
+constexpr int SYM2_MINCTAS = 7;
 constexpr uint32_t SYM2_UNITS = SYM_SMEM_UNITS + 2 * 2 + 2 * 1;            // uint4 per group
 constexpr uint32_t SYM2_ABORT = 1u << 8, SYM2_IDS = 1u << 9, SYM2_MODE = 1u << 10;
 
-template <int R, bool SPLIT = false>
+template <int R>
 struct SymGroup {
-  static constexpr uint32_t STRIDE = SPLIT ? SYM2_GROUPS : SYM_LANES;   // columns of the CTA's per-group shared memory
+  static constexpr uint32_t STRIDE = SYM2_GROUPS;   // columns of the CTA's per-group shared memory
   const Dev& d;
   const uint32_t g;
   const size_t plane;
@@ -114,15 +112,13 @@ struct SymGroup {
     const uint4 e = slot(r, bid);
     if (e.x == bid) { next = e.y; tok = (uint64_t)e.z | ((uint64_t)e.w << 32); return; }
     next = __ldcg(d.cnext + row(r, bid));   // rows written earlier in this launch by this lane: read them at L2
-    tok = __ldcg(d.ctok + row(r, bid));
-    if (!SPLIT) cache_put(r, bid, next, tok);   // (split kernel: a cache is only written at entry and by appends, see fetch_sent)
+    tok = __ldcg(d.ctok + row(r, bid));     // (a miss does not fill: a cache is only written at entry and by appends, see fetch_sent)
   }
-  // sym2_kernel, follower lane: a block the leader sent one tick ago, read from the LEADER's row cache, which the leader
-  // lane is appending to right now.  Its appends of this tick are the ids (mk_sent, mk_sent + n_app]; a slot one of them
-  // maps to is not read (the row is in global memory, written before the last barrier).  No other write happens to that
-  // cache after entry, so every slot this reads is quiescent.
+  // Follower lane: a block the leader sent one tick ago, read from the LEADER's row cache, which the leader lane is
+  // appending to right now.  Its appends of this tick are the ids (mk_sent, mk_sent + n_app]; a slot one of them maps to
+  // is not read (the row is in global memory, written before the last barrier).  No other write happens to that cache
+  // after entry, so every slot this reads is quiescent.
   __device__ __forceinline__ void fetch_sent(uint32_t bid, uint32_t mk_sent, uint32_t n_app, uint32_t& next, uint64_t& tok) {
-    if (!SPLIT) { fetch(L, bid, next, tok); return; }
     if (!in_window(bid)) { next = ABSENT; tok = 0; return; }
     if (bid + SYM_ROWS > mk_sent + n_app) {
       const uint4 e = slot(L, bid);
@@ -326,14 +322,12 @@ struct SymGroup {
     }
     out.ae = 1;                                            // replicate() follows: one AppendEntries per peer
     out.mk = maxkey;
-    if (!SPLIT) replicate(ph_f, mode_f, maxkey, out);
   }
   // replicate, leader.rs:124-174: Probe -> range(head..).nth(1); Replicate -> range(head..).skip(1).take(5), over the
-  // leader's table as it stood when its largest key was `mk`.  The one-lane kernel runs it inside the leader's tick.  In
-  // sym2_kernel the FOLLOWER lane runs the same scan at the start of the next tick (follower_tick_view), from the
-  // {progress head, mode, max key} the leader lane put in its mail -- the same rows, read through fetch_sent, the same
-  // blocks; it takes a sixth of the leader's chain off the critical lane.  (The leader lane runs this once itself, for
-  // the outbox the launch leaves behind.)
+  // leader's table as it stood when its largest key was `mk`.  Within the launch the FOLLOWER lane runs this scan at the
+  // start of the next tick (follower_tick_view), from the {progress head, mode, max key} the leader lane put in its mail
+  // -- the same rows, read through fetch_sent, the same blocks; it takes a sixth of the leader's chain off the critical
+  // lane.  The leader lane runs it once itself, after the last tick, for the outbox the launch leaves behind.
   __device__ __forceinline__ void replicate(uint32_t phf, uint32_t modef, uint32_t mk, SymMail& out) {
     const uint32_t take = modef ? JR_MAX_AE_BLOCKS : 1u;
     uint32_t bid = max(phf, tbase), pulled = 0, nb = 0;
@@ -402,7 +396,7 @@ struct SymGroup {
     }
     // Command::Tick: the election timer cannot have expired (sym_enter checked the bound)
   }
-  // sym2_kernel, follower lane: the same tick when the AppendEntries' blocks are not listed in the mail.  The leader's
+  // Follower lane: the same tick when the AppendEntries' blocks are not listed in the mail.  The leader's
   // replicate() (leader.rs:124-174: Probe -> range(head..).nth(1); Replicate -> range(head..).skip(1).take(5)) is run
   // HERE, over the leader's table as it stood when its largest key was `mk`, and each block it yields is applied on the
   // spot -- the same blocks in the same order as listing them first, without the list and without reading them twice.
@@ -435,8 +429,8 @@ struct SymGroup {
 };
 
 // ---- entry: is the group symmetric, is its mail canonical? ---------------------------------------------------------
-template <int R, bool SPLIT>
-__device__ __forceinline__ bool sym_enter(SymGroup<R, SPLIT>& s, SymMail& m, const StepParams& p, int prv) {
+template <int R>
+__device__ __forceinline__ bool sym_enter(SymGroup<R>& s, SymMail& m, const StepParams& p, int prv) {
   const Dev& d = s.d;
   if (s.g >= d.G) return false;
   // roles: one live leader, R-1 live followers of that leader
@@ -639,8 +633,8 @@ __device__ __forceinline__ bool sym_enter(SymGroup<R, SPLIT>& s, SymMail& m, con
 }
 
 // ---- exit: write everything step_kernel would have left behind -------------------------------------------------------
-template <int R, bool SPLIT>
-__device__ __forceinline__ void sym_leave_leader(SymGroup<R, SPLIT>& s, const SymMail& last, int cur_last) {
+template <int R>
+__device__ __forceinline__ void sym_leave_leader(SymGroup<R>& s, const SymMail& last, int cur_last) {
   const Dev& d = s.d;
   const uint32_t L = s.L;
   {  // leader: P2, P3, progress planes, max key (P0 / P1 are untouched by a steady leader)
@@ -690,8 +684,8 @@ __device__ __forceinline__ void sym_leave_leader(SymGroup<R, SPLIT>& s, const Sy
   }
 }
 
-template <int R, bool SPLIT>
-__device__ __forceinline__ void sym_leave_followers(SymGroup<R, SPLIT>& s, const SymMail& last, int cur_last) {
+template <int R>
+__device__ __forceinline__ void sym_leave_followers(SymGroup<R>& s, const SymMail& last, int cur_last) {
   const Dev& d = s.d;
   const uint32_t L = s.L;
   // The followers emitted the same Instructions.  If none of them has anything pending since the last drain, ONE set of
@@ -727,85 +721,13 @@ __device__ __forceinline__ void sym_leave_followers(SymGroup<R, SPLIT>& s, const
   }
 }
 
-// One lane per group.  symdone[g] = 1: the whole launch of group g has been applied here; 0: step_kernel runs it.
-template <int R>
-__global__ void __launch_bounds__(SYM_LANES, 512 / SYM_LANES) sym_kernel(const Dev d, const StepParams p, uint8_t* symdone) {
-  const uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;
-  if (g >= d.Gp) return;
-  SymGroup<R> s(d, g);
-  SymMail a, b;
-  s.abort = false;
-  s.lcnt = s.fcnt = 0;
-  s.n_hb = 0;
-  s.last_hb = 0;
-  s.share = false;
-  s.n_app = 1u + p.n_synth;
-  __shared__ uint4 lane_smem[SYM_SMEM_UNITS * SYM_LANES];
-  s.rows = lane_smem + threadIdx.x;
-  s.enc = lane_smem + 2 * SYM_ROWS * SYM_LANES + threadIdx.x;
-  s.cache_clear();
-  bool ok = sym_enter(s, a, p, 1 - p.cur);
-  if (ok) {
-    s.cache_fill(s.L, s.maxkey);
-    s.cache_fill(s.F0, s.fmaxkey);
-    s.share = (d.flags & JR_F_CAPTURE_FSM) != 0;
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-      if ((uint32_t)r == s.L) continue;
-      const uint2 c = d.fc[s.rg(r)];
-      if (c.x | c.y) s.share = false;
-    }
-    s.enc_init_leader((d.flags & JR_F_CAPTURE_FSM) ? d.fc[s.rg(s.L)] : make_uint2(0u, 0u));
-    s.enc_init_followers();
-    const jr_proposal* props = p.proposals;
-    s.now = p.now;
-    for (uint32_t t = 0; t < p.n_ticks && !s.abort; ++t) {
-      b = SymMail{};
-      uint64_t tok = 0;
-      if ((p.phases & PH_PROPOSE) && (props || p.tok_runs)) {
-        uint4 pr;
-        if (p.tok_runs) {
-          const uint4 rn = __ldg(p.tok_runs + g);
-          const uint64_t base = (uint64_t)rn.x | ((uint64_t)rn.y << 32);
-          const uint64_t tk = base + (uint64_t)(p.tok_tick + t) * ((uint64_t)rn.z | ((uint64_t)rn.w << 32));
-          pr = make_uint4((uint32_t)tk, (uint32_t)(tk >> 32), base ? __ldg(p.tok_route + g) : 0u, 0u);
-        } else {
-          pr = __ldg(reinterpret_cast<const uint4*>(props) + g);
-          props += p.prop_stride;
-        }
-        if (pr.z == s.L + 1) tok = (uint64_t)pr.x | ((uint64_t)pr.y << 32);
-        else if (pr.z != 0) s.abort = true;               // a proposal for a follower: proxied ClientRequest, not canonical
-      }
-      if (s.abort) break;
-      s.leader_tick(a, b, tok, (p.phases & PH_PROPOSE) ? p.n_synth : 0u, p.step_index + t);
-      if (s.abort) break;
-      s.follower_tick(a, b);
-      a = b;
-      s.now += p.dt;
-    }
-    ok = !s.abort;
-    if (ok) {
-      const int cur_last = p.cur ^ (int)((p.n_ticks - 1) & 1u);
-      sym_leave_leader(s, a, cur_last);
-      sym_leave_followers(s, a, cur_last);
-    }
-  }
-  symdone[g] = ok ? 1 : 0;
-}
-
 // Two lanes per group (see SYM2_GROUPS above).  Both lanes run sym_enter on the same, still untouched planes and reach
 // the same verdict; afterwards each keeps to its side: the leader lane owns the leader's table cache, encoder state,
 // planes and outbox, the follower lane those of the followers.  Either side may abort: it says so in its mail, the
 // other side sees it one barrier later, and after the last barrier both check the other's final mail, so a group is
 // either left (by both) or not at all.
-#ifndef JR_SYM2_MINCTAS
-#define JR_SYM2_MINCTAS 7
-#endif
-#ifndef JR_SYM2_ROLES
-#define JR_SYM2_ROLES 3   // (register-need experiments: 1 = leader code only, 2 = follower code only)
-#endif
 template <int R>
-__global__ void __launch_bounds__(2 * SYM2_GROUPS, JR_SYM2_MINCTAS) sym2_kernel(const Dev d, const StepParams p, uint8_t* symdone, uint8_t* symblk) {
+__global__ void __launch_bounds__(2 * SYM2_GROUPS, SYM2_MINCTAS) sym2_kernel(const Dev d, const StepParams p, uint8_t* symdone, uint8_t* symblk) {
   JR_DYN_SMEM(uint4, smem);
   // One __syncthreads() per tick for both warp pairs of the CTA.  (A named barrier per pair -- `bar.sync 0/1, 64`, the
   // pairs never need each other -- measured 3% SLOWER, twice; with a register operand for the id ptxas charges the CTA
@@ -816,7 +738,7 @@ __global__ void __launch_bounds__(2 * SYM2_GROUPS, JR_SYM2_MINCTAS) sym2_kernel(
   const bool lead = ((w ^ blockIdx.x) & 1u) == 0;          // roles alternate from CTA to CTA: no SM sub-partition gets leaders only
   const uint32_t gi = (w >> 1) * 32u + lane;               // group within the CTA
   const uint32_t g = blockIdx.x * S + gi;                  // (g >= Gp: sym_enter says no; the lane only keeps the barriers company)
-  SymGroup<R, true> s(d, g);
+  SymGroup<R> s(d, g);
   s.abort = false;
   s.lcnt = s.fcnt = 0;
   s.n_hb = 0;
@@ -858,7 +780,7 @@ __global__ void __launch_bounds__(2 * SYM2_GROUPS, JR_SYM2_MINCTAS) sym2_kernel(
   s.now = p.now;
   uint32_t cur = 0;                                        // mail buffer written this tick; 1 - cur is read
   for (uint32_t t = 0; t < p.n_ticks; ++t) {
-    if (lead && (JR_SYM2_ROLES & 1)) {
+    if (lead) {
       if (!dead) {
         const uint4 c = mail[(4 + (1 - cur)) * S];
         if (c.x & SYM2_ABORT) dead = true;
@@ -889,7 +811,7 @@ __global__ void __launch_bounds__(2 * SYM2_GROUPS, JR_SYM2_MINCTAS) sym2_kernel(
         }
       }
       if (dead) mail[(2 * cur) * S] = make_uint4(SYM2_ABORT, 0u, 0u, 0u);
-    } else if (!lead && (JR_SYM2_ROLES & 2)) {
+    } else {
       if (!dead) {
         const uint4 ma = mail[(2 * (1 - cur)) * S];
         if (ma.x & SYM2_ABORT) dead = true;
@@ -953,16 +875,6 @@ __global__ void __launch_bounds__(2 * SYM2_GROUPS, JR_SYM2_MINCTAS) sym2_kernel(
       if (g < d.G) *(volatile uint32_t*)d.hunf = p.epoch;   // advisory, for the host's choice of the next step_kernel grid
     }
   }
-}
-
-// symblk[b] = every group of 32-group block b was folded (step_kernel CTAs of such blocks return at once)
-__global__ void sym_blocks_kernel(const uint8_t* symdone, uint8_t* symblk, uint32_t n_blocks) {
-  const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b >= n_blocks) return;
-  const uint4* v = reinterpret_cast<const uint4*>(symdone + (size_t)b * GROUPS_PER_CTA);
-  const uint4 x = v[0], y = v[1];
-  const uint32_t all = 0x01010101u;
-  symblk[b] = (x.x == all && x.y == all && x.z == all && x.w == all && y.x == all && y.y == all && y.z == all && y.w == all) ? 1 : 0;
 }
 
 #endif  // JR_DEVICE_CODE

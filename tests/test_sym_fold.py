@@ -1,8 +1,8 @@
 """The symmetric-group fold (josefine_b200/csrc/sym_fold.cuh): jr_run* applies a whole launch of a symmetric group in
-one lane.  It must be indistinguishable from step_kernel: replica state, block tables, leader tables and Instruction
-streams equal those of an engine that never folds (JR_F_NO_SYMMETRIC_FOLD) AND those of the oracle.  (Engines with
-JR_F_STREAM_DIGEST never fold, so the digest-based parity suites keep testing step_kernel; here everything except
-the Message stream is compared.)"""
+two lanes of sym2_kernel, one for the leader and one standing for every follower.  It must be indistinguishable from
+step_kernel: replica state, block tables, leader tables and Instruction streams equal those of an engine that never
+folds (JR_F_NO_SYMMETRIC_FOLD) AND those of the oracle.  (Engines with JR_F_STREAM_DIGEST never fold, so the
+digest-based parity suites keep testing step_kernel; here everything except the Message stream is compared.)"""
 import pytest
 
 from josefine_b200 import abi, Command, fsm_tuple
@@ -334,12 +334,4 @@ def test_random_scripts_on_device_code(seed):
 @pytest.mark.parametrize("seed", [100, 101, 102, 103])
 def test_random_scripts_on_gpu(seed):
     folded_any, _ = _random_script(_gpu, seed, rounds=12)
-    assert folded_any
-
-
-@pytest.mark.parametrize("seed", [3, 8])
-def test_random_scripts_one_lane_kernel_on_device_code(seed, monkeypatch):
-    """The one-lane sym_kernel (JR_SYM_ONE_LANE=1: A/B and fallback) obeys the same contract."""
-    monkeypatch.setenv("JR_SYM_ONE_LANE", "1")
-    folded_any, _ = _random_script(_emu, seed)
     assert folded_any

@@ -54,13 +54,4 @@ for R, G in ((3, 70), (5, 96)):
     e.node_restart(0, 2, now, blocks, int(e.query(0, 2).commit))
     e.run(now, 100, 6, 1)
     print(R, "folded per launch", folded, e.state_digest(), e.fault_count())
-# the one-lane fold (A/B and fallback path) once as well
-os.environ["JR_SYM_ONE_LANE"] = "1"
-e = RaftEngine.create(64, 5, seed=5, flags=abi.F_CAPTURE_FSM, chain_capacity=64, fsm_units=32)
-e.step(0, flags=0, inject=bootstrap(64, 5))
-for rnd in range(3):
-    e.run(100 + 2000 * rnd, 100, 20, 1)
-    e.truncate(4)
-    e.fsm_records()
-print("one-lane fold", e.fold_count(), e.state_digest(), e.fault_count())
 print("round-2 sanitize workload done")

@@ -17,9 +17,10 @@ from josefine_b200 import abi  # noqa: E402
 EXPLICIT_TRUNCATE = False
 
 
-def measure(bn, label, G, R, steps, capture=True, flush=True, **kw):
+def measure(bn, label, G, R, steps, capture=True, flush=True, fold=True, **kw):
     torch = bn.torch
-    eng = bn.steady_engine(G, R, abi.F_CAPTURE_FSM if capture else 0, auto_truncate=not EXPLICIT_TRUNCATE, **kw)
+    flags = (abi.F_CAPTURE_FSM if capture else 0) | (0 if fold else abi.F_NO_SYMMETRIC_FOLD)
+    eng = bn.steady_engine(G, R, flags, auto_truncate=not EXPLICIT_TRUNCATE, **kw)
     lib, h = eng._lib, eng._h
     S = bench.TICKS_PER_STEP
     now = bench.DT_MS * 17
@@ -77,11 +78,9 @@ def main():
     G, R = bench.GROUPS_PER_GPU, bench.REPLICAS
     variants = [("headline", G, {}), ("headline, no capture", G, {"capture": False}), ("scattered leaders", G, {"scattered": True}),
                 ("headline, warm L2 (no flush)", G, {"flush": False}), ("heartbeat every tick", G, {"heartbeat_ms": 99}),
-                ("131,072 groups", 2 * G, {}), ("headline, fold off (step_kernel)", G, {"_nofold": True}),
-                ("no capture, fold off", G, {"capture": False, "_nofold": True})]
+                ("131,072 groups", 2 * G, {}), ("headline, fold off (step_kernel)", G, {"fold": False}),
+                ("no capture, fold off", G, {"capture": False, "fold": False})]
     for label, g, kw in variants[:a.only]:
-        if kw.pop("_nofold", False):
-            os.environ["JR_NO_FOLD"] = "1"
         measure(bn, label, g, R, a.steps, **kw)
 
 
