@@ -171,7 +171,7 @@ typedef struct jr_config {
                                 * nodes are never stepped, and mail addressed to them is only
                                 * returned through out_msgs for the host to forward.           */
   uint32_t fsm_host_records;   /* records one jr_fsm_records_async batch may hold (pinned host memory,
-                                * JR_STAGING_DEPTH buffers of this size); 0 = max(3 * n_groups * n_replicas + 1024,
+                                * JR_STAGING_DEPTH + 1 buffers of this size); 0 = max(3 * n_groups * n_replicas + 1024,
                                 * min(n_groups * n_replicas * fsm_units, 65536))                            */
   uint32_t fsm_raw_units;      /* scratch: raw Instructions one replica may emit per launch before they are encoded into
                                 * records at the launch's end; 0 = 192.  jr_run* cut their work into launches of at most
@@ -428,10 +428,10 @@ jr_status jr_drain_fsm(jr_engine* e, jr_fsm_instr* out, size_t cap, size_t* n);
 /*
  * The batched output path.  jr_fsm_records_async ENQUEUES, after everything submitted so far: pack all records
  * accumulated since the last drain into one dense array sorted by (node, group) and write it to the engine's
- * next pinned host buffer (JR_STAGING_DEPTH = 3 buffers, filled by the copy engine: the SMs stay with the next
- * step).  The FIFOs are empty afterwards.  jr_fsm_records_wait blocks until the OLDEST outstanding batch has landed
- * and returns it: `*records` points into the engine's buffer and stays valid until the JR_STAGING_DEPTH-1'th
- * jr_fsm_records_async call after this one.  JR_E_CAPACITY (batch still returned) if records were dropped.  At
+ * next pinned host buffer (JR_STAGING_DEPTH + 1 = 4 buffers used in turn, filled by the copy engine: the SMs stay with
+ * the next step).  The FIFOs are empty afterwards.  jr_fsm_records_wait blocks until the OLDEST outstanding batch has
+ * landed and returns it: `*records` points into the engine's buffer and stays valid until the JR_STAGING_DEPTH-1'th
+ * jr_fsm_records_async call after this one, also when JR_STAGING_DEPTH batches were outstanding before the wait.  JR_E_CAPACITY (batch still returned) if records were dropped.  At
  * most JR_STAGING_DEPTH batches may be outstanding.  Requires JR_F_CAPTURE_FSM.
  * Threads: an engine is driven by ONE submitting thread (josefine's event_loop task); jr_fsm_records_wait and
  * jr_leader_table_wait (and the pure host functions jr_fsm_expand / jr_fsm_fold*) may be called from ONE other thread at

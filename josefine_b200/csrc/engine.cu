@@ -766,15 +766,21 @@ struct jr_engine {
   void* many_buf = nullptr;
   size_t many_cap = 0;
   // Instruction-stream drain (JR_F_CAPTURE_FSM): scan -> pack into stage[b] on the engine stream, then
-  // the copy engine moves stage[b] into the pinned host buffer host[b] on the d2h stream.
+  // the copy engine moves stage[b] into the pinned host buffer host[fsm_host_of[b]] on the d2h stream.
+  // The host buffers rotate on their own, one more of them than stage buffers: with NBUF batches outstanding, the
+  // async right after a wait must not land in the buffer that wait has just returned (it stays the caller's until
+  // the NBUF-1'th async after the wait, include/josefine_raft_abi.h).
+  static constexpr int NHOST = NBUF + 1;
   unsigned long long* fsm_part = nullptr;                     // device, 3 x (CTAs of the count/pack kernels): per-CTA sums -> offsets
   uint32_t fsm_cap = 0;                                       // records per batch
   uint4* fsm_stage[NBUF] = {nullptr, nullptr};                // device, 2 * fsm_cap uint4 each
   FsmHeader* fsm_stage_hdr[NBUF] = {nullptr, nullptr};        // device
-  uint4* fsm_host[NBUF] = {nullptr, nullptr};                 // pinned + mapped host
+  uint4* fsm_host[NHOST] = {nullptr, nullptr};                // pinned + mapped host
+  int fsm_host_of[NBUF] = {0, 0};                             // host buffer the batch in stage[b] lands in
+  int fsm_hi = 0;                                             // next host buffer
   FsmHeader* fsm_host_hdr[NBUF] = {nullptr, nullptr};         // pinned + mapped host
   cudaEvent_t fsm_packed[NBUF] = {nullptr, nullptr};          // pack into stage[b] finished (engine stream)
-  cudaEvent_t fsm_landed[NBUF] = {nullptr, nullptr};          // copy into host[b] finished (d2h stream)
+  cudaEvent_t fsm_landed[NBUF] = {nullptr, nullptr};          // copy of stage[b] to the host finished (d2h stream)
   size_t fsm_copied[NBUF] = {0, 0};                           // records of stage[b] the enqueued copy covers
   size_t fsm_last_records = 0;                                // size of the last batch taken (the next copy's guess)
   bool fsm_used[NBUF] = {false, false};
@@ -1072,9 +1078,10 @@ jr_status jr_engine_create(const jr_config* cfg, jr_engine** out) {
            cudaEventCreateWithFlags(&e->batch_free[i], cudaEventDisableTiming) == cudaSuccess &&
            cudaEventCreateWithFlags(&e->fsm_packed[i], cudaEventDisableTiming) == cudaSuccess &&
            cudaEventCreateWithFlags(&e->fsm_landed[i], cudaEventDisableTiming) == cudaSuccess;
-    for (int i = 0; ok && e->fsm_cap && i < jr_engine::NBUF; ++i)   // the drain's landing buffers: pinned, device-visible
-      ok = cudaHostAlloc((void**)&e->fsm_host[i], (size_t)e->fsm_cap * sizeof(jr_fsm_record), cudaHostAllocMapped) == cudaSuccess &&
-           cudaHostAlloc((void**)&e->fsm_host_hdr[i], sizeof(FsmHeader), cudaHostAllocMapped) == cudaSuccess;
+    for (int i = 0; ok && e->fsm_cap && i < jr_engine::NHOST; ++i)   // the drain's landing buffers: pinned, device-visible
+      ok = cudaHostAlloc((void**)&e->fsm_host[i], (size_t)e->fsm_cap * sizeof(jr_fsm_record), cudaHostAllocMapped) == cudaSuccess;
+    for (int i = 0; ok && e->fsm_cap && i < jr_engine::NBUF; ++i)
+      ok = cudaHostAlloc((void**)&e->fsm_host_hdr[i], sizeof(FsmHeader), cudaHostAllocMapped) == cudaSuccess;
     if (!ok) {
       set_err("copy streams / events could not be created");
       jr_engine_destroy(e);
@@ -1175,11 +1182,12 @@ void jr_engine_destroy(jr_engine* e) {
     if (e->batch_free[i]) cudaEventDestroy(e->batch_free[i]);
     if (e->fsm_packed[i]) cudaEventDestroy(e->fsm_packed[i]);
     if (e->fsm_landed[i]) cudaEventDestroy(e->fsm_landed[i]);
-    if (e->fsm_host[i]) cudaFreeHost(e->fsm_host[i]);
     if (e->fsm_host_hdr[i]) cudaFreeHost(e->fsm_host_hdr[i]);
     if (e->batch[i]) cudaFree(e->batch[i]);
     if (e->tokbuf[i]) cudaFree(e->tokbuf[i]);
   }
+  for (int i = 0; i < jr_engine::NHOST; ++i)
+    if (e->fsm_host[i]) cudaFreeHost(e->fsm_host[i]);
   if (e->h_scatter) cudaFreeHost((void*)e->h_scatter);
   if (e->h_unfolded) cudaFreeHost((void*)e->h_unfolded);
   if (e->own_stream) cudaStreamDestroy(e->own_stream);
@@ -1284,8 +1292,10 @@ static jr_status fsm_records_enqueue(jr_engine* e) {
     if (e->fsm_npending == jr_engine::NBUF) { set_err("%d batches outstanding: call jr_fsm_records_wait first", jr_engine::NBUF); return JR_E_INVAL; }
     last_records = e->fsm_last_records;
   }
-  const int b = e->fsm_i;
+  const int b = e->fsm_i, hb = e->fsm_hi;
   e->fsm_i = (b + 1) % jr_engine::NBUF;
+  e->fsm_hi = (hb + 1) % jr_engine::NHOST;
+  e->fsm_host_of[b] = hb;
   const size_t plane = (size_t)d.R * d.Gp;
   if (e->fsm_used[b]) CK(cudaStreamWaitEvent(e->stream, e->fsm_landed[b], 0));  // stage[b] has left the device
 #ifdef JR_EMU
@@ -1307,7 +1317,7 @@ static jr_status fsm_records_enqueue(jr_engine* e) {
   // (A copy by the SMs would store to host memory through the LSUs the next step's kernel needs: that kernel is one wave
   // of CTAs, so the slowest SM sets its duration.  A DMA copy takes nothing from the SMs.)
   const size_t guess = std::min<size_t>(e->fsm_cap, std::max<size_t>(last_records + last_records / 8 + 1024, 16384));
-  if (guess) CK(cudaMemcpyAsync(e->fsm_host[b], e->fsm_stage[b], guess * sizeof(jr_fsm_record), cudaMemcpyDeviceToHost, e->d2h));
+  if (guess) CK(cudaMemcpyAsync(e->fsm_host[hb], e->fsm_stage[b], guess * sizeof(jr_fsm_record), cudaMemcpyDeviceToHost, e->d2h));
   CK(cudaMemcpyAsync(e->fsm_host_hdr[b], e->fsm_stage_hdr[b], sizeof(FsmHeader), cudaMemcpyDeviceToHost, e->d2h));
   e->fsm_copied[b] = guess;
   CK(cudaEventRecord(e->fsm_landed[b], e->d2h));
@@ -1322,22 +1332,28 @@ static jr_status fsm_records_take(jr_engine* e, const jr_fsm_record** recs, jr_f
   {
     std::lock_guard<std::mutex> l(e->qmu);
     if (e->fsm_npending == 0) { set_err("no batch outstanding"); return JR_E_INVAL; }
-    b = e->fsm_pending[0];
-    for (int k = 0; k + 1 < jr_engine::NBUF; ++k) e->fsm_pending[k] = e->fsm_pending[k + 1];
-    --e->fsm_npending;
+    b = e->fsm_pending[0];   // (only this thread removes entries: the oldest stays b while the submitting thread appends)
   }
+  uint4* host = e->fsm_host[e->fsm_host_of[b]];
   CK(cudaEventSynchronize(e->fsm_landed[b]));
-  const FsmHeader& h = *e->fsm_host_hdr[b];
+  const FsmHeader h = *e->fsm_host_hdr[b];   // a copy: once stage[b] is released below, the next batch's header lands there
   if (h.n_records > e->fsm_copied[b]) {   // the speculative copy was short: fetch the tail now (stage[b] is still intact)
     const size_t have = e->fsm_copied[b];
-    CK(cudaMemcpyAsync(reinterpret_cast<jr_fsm_record*>(e->fsm_host[b]) + have, reinterpret_cast<const jr_fsm_record*>(e->fsm_stage[b]) + have,
+    CK(cudaMemcpyAsync(reinterpret_cast<jr_fsm_record*>(host) + have, reinterpret_cast<const jr_fsm_record*>(e->fsm_stage[b]) + have,
                        ((size_t)h.n_records - have) * sizeof(jr_fsm_record), cudaMemcpyDeviceToHost, e->d2h));
     CK(cudaEventRecord(e->fsm_landed[b], e->d2h));
     CK(cudaEventSynchronize(e->fsm_landed[b]));
     e->fsm_copied[b] = h.n_records;
   }
-  { std::lock_guard<std::mutex> l(e->qmu); e->fsm_last_records = h.n_records; }
-  if (recs) *recs = reinterpret_cast<const jr_fsm_record*>(e->fsm_host[b]);
+  {
+    // Only now is stage[b] free for the next jr_fsm_records_async: until the tail above had landed, a pack into it from
+    // the submitting thread would have overwritten records not yet copied out.
+    std::lock_guard<std::mutex> l(e->qmu);
+    for (int k = 0; k + 1 < jr_engine::NBUF; ++k) e->fsm_pending[k] = e->fsm_pending[k + 1];
+    --e->fsm_npending;
+    e->fsm_last_records = h.n_records;
+  }
+  if (recs) *recs = reinterpret_cast<const jr_fsm_record*>(host);
   if (batch) {
     memset(batch, 0, sizeof *batch);
     batch->n_records = h.n_records;
